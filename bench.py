@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — CFR iterations/s of the B200 engine on BASELINE.json's workloads.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload config4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload config4] [--dump-outputs DIR]
 
 Default workload: config 4 (flop-rooted subgame, 49 turn cards x 48 river cards = 2 352 river boards, 29 GB of infoset
 tables: the largest configuration that fits one B200 and the one north_star names for board sharding).  The same run
@@ -13,14 +13,17 @@ the workload.  N > 1 is launched by torchrun, one rank per GPU; the first dealt-
 the counterfactual values at the shared chance nodes are exchanged every traversal inside the traversal kernel over
 NVLink peer memory (strong scaling: the job is the same subgame at every N; config 5 shards by subgame, no exchange).
 
-Rank 0 prints ONE JSON line (keys documented in the task contract): value = iterations/s with all inputs resident in
-HBM (CUDA events around each step, L2 flushed between steps, max over ranks; the K-step timed region is repeated until
-it has run for at least 2 s and the median repetition is reported), e2e = the same through the C ABI from host
+Rank 0 prints ONE JSON line: value = iterations/s with all inputs resident in HBM (CUDA events around each of the K
+timed steps, L2 flushed between steps, max over ranks), e2e = the same through the C ABI from host
 buffers, roofline = the dominant kernel (one launch per player traversal) from CUDA events on the engine's stream,
 cpu_baseline = the literal scalar port of the reference's cfr() on this box's host cores (plus, for context, the
 vector-form fp64 oracle and the literal 8-thread mccfr port).
 `--impl reference` times that port alone (the reference itself cannot be built: no Rust toolchain); it rebuilds the
 workload from tests/golden/workload_*.npz and oracle/tree_oracle.py and never loads the product library.
+
+`--dump-outputs DIR` (one GPU) writes what the engine holds after the last timed step of the main workload, i.e. after
+exactly W + K iterations from zero tables, as float .npy files (see collect_outputs).  The inputs are fixed by the
+workload, so two builds run with the same arguments can be compared array by array.
 """
 from __future__ import annotations
 
@@ -43,7 +46,8 @@ METRIC = "cfr_iterations_per_sec"
 UNIT = "iter/s"
 BYTES_PER_UPDATE = 20  # SURVEY §8(d): regret R+W (8) + strategy_sum R+W (8) + opponent-side regret read (4)
 BB_CHIPS = 1.0         # the reference has no big blind (options.rs:10-28): mbb/g is quoted for a big blind of 1 chip
-MIN_TIMED_SECONDS = 2.0
+DUMP_BYTES = 60_000_000  # arrays of --dump-outputs: with their .npy headers below 64 MB
+DUMP_SEED = 20240601
 
 
 def load_peaks():
@@ -216,7 +220,7 @@ def run_reference(args):
     if rank != 0:
         return 0
     set_host_threads()
-    steps, warmup = max(1, args.steps), max(0, args.warmup)
+    steps, warmup = args.steps, args.warmup
     target = min(8.0, 150.0 / (steps + warmup))  # the whole run stays within a few minutes whatever K and W are
     rate, t_step, cores, sample, upd = cpu_port_rate(args.workload, target, steps, warmup)
     line = {
@@ -240,8 +244,67 @@ class Ctx:
     pass
 
 
-def measure(cx, name: str, steps: int, warmup: int, min_seconds: float, with_clocks: bool):
-    """Device-resident throughput, end-to-end throughput and the per-kernel roofline of one workload."""
+def _dealt_cards(i: int, live, k: int):
+    """The i-th deal, in lexicographic order, of k cards one after another from `live`."""
+    rest, out = list(live), []
+    for j in range(k):
+        q, i = divmod(i, int(np.prod([len(rest) - 1 - t for t in range(k - 1 - j)])))
+        out.append(rest.pop(q))
+    return out
+
+
+def collect_outputs(eng, w, tree, ranges) -> dict:
+    """What a caller of rs_iterate reads back, keyed by what the caller supplies (hand slots of its ranges, dealt
+    cards) rather than by the engine's row and board numbering:
+      root_values_p0/_p1   [root boards, hands]   rs_root_values: counterfactual values of the last traversal
+      regrets/strategy_sum [S, hands, actions]    rs_read_infoset row of each hand slot (card table); 0 where the
+                                                  hand hits the board (it has no reach), past the player's range or
+                                                  past the node's actions
+      slab_keys            [S, 4]                 action node index, its number of actions, then the cards dealt
+                                                  beyond the root board (the subgame for a batch); -1 where unused
+    The S slabs are a fixed seeded sample of all (action node, board) pairs: as many as DUMP_BYTES leaves room for."""
+    st = eng.stats()
+    out = {f"root_values_p{p}": eng.root_values(p) for p in range(2)}
+    nodes = [i for i in range(tree.n_nodes) if tree.type[i] == 0]
+    rounds = [int(tree.round_idx[i]) for i in nodes]
+    counts = np.array([st.n_boards[k] for k in rounds], dtype=np.int64)
+    first = np.cumsum(counts) - counts
+    live = [c for c in range(52) if not (w.options.board_mask >> c) & 1]
+    H, A = max(len(r) for r in ranges), max(len(tree.children_of(i)) for i in nodes)
+    room = DUMP_BYTES - sum(a.nbytes for a in out.values())
+    n = int(min(counts.sum(), room // (2 * 4 * H * A + 4 * 8)))
+    pick = np.sort(np.random.default_rng(DUMP_SEED).choice(int(counts.sum()), n, replace=False))
+    regrets = np.zeros((n, H, A), dtype=np.float32)
+    ssum = np.zeros((n, H, A), dtype=np.float32)
+    keys = np.full((n, 4), -1.0)
+    for s, flat in enumerate(pick):
+        j = int(np.searchsorted(first, flat, side="right")) - 1
+        node, k, b = nodes[j], rounds[j], int(flat - first[j])
+        if w.board_masks is not None:  # a batch: subgame b is board b of round 0
+            keys[s, 2] = b
+        else:
+            dealt = _dealt_cards(b, live, k)
+            keys[s, 2:2 + k] = dealt
+            b = eng.board_id(k, dealt)
+        rows = eng.card_table(k, int(tree.player[node]), b)
+        r, sm = eng.read_infoset(int(tree.an_index[node]), b)
+        keys[s, :2] = int(tree.an_index[node]), r.shape[1]
+        hands = np.flatnonzero(rows != 0xFFFF)
+        regrets[s, hands, :r.shape[1]] = r[rows[hands]]
+        ssum[s, hands, :r.shape[1]] = sm[rows[hands]]
+    out.update(regrets=regrets, strategy_sum=ssum, slab_keys=keys)
+    return out
+
+
+def write_outputs(d: Path, arrays: dict):
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", a)
+
+
+def measure(cx, name: str, steps: int, warmup: int, with_clocks: bool, dump_dir=None):
+    """Device-resident throughput, end-to-end throughput and the per-kernel roofline of one workload; with `dump_dir`,
+    the outputs of the last timed step are written there."""
     import torch
     import torch.distributed as dist
     import rustsolver_b200 as rb
@@ -280,8 +343,7 @@ def measure(cx, name: str, steps: int, warmup: int, min_seconds: float, with_clo
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    # ---- device-resident throughput: K steps, each bracketed by the engine's own CUDA events; the K-step region is
-    # repeated until it has run for min_seconds in total and the median repetition is reported ----
+    # ---- device-resident throughput: K steps, each bracketed by the engine's own CUDA events ----
     for _ in range(warmup):
         eng.iterate(1)
     sampler = ClockSampler(cx.local_rank) if with_clocks else None
@@ -289,26 +351,20 @@ def measure(cx, name: str, steps: int, warmup: int, min_seconds: float, with_clo
     if sampler:
         sampler.start()
     wall0 = time.perf_counter()
-    reps, launches = [], 0
-    while True:
-        ms_before = eng.stats().device_ms
-        l_before = eng.stats().kernel_launches
-        for _ in range(steps):
-            cx.flush_l2()
-            barrier()
-            eng.iterate(1)  # rs_iterate records events on its launch stream around the graph replay
+    s0 = eng.stats()
+    for _ in range(steps):
+        cx.flush_l2()
         barrier()
-        s1 = eng.stats()
-        reps.append(max_over_ranks(s1.device_ms - ms_before))
-        launches = int(s1.kernel_launches - l_before)
-        done = max_over_ranks(1.0 if (time.perf_counter() - wall0 >= min_seconds or len(reps) >= 50) else 0.0)
-        if done > 0:
-            break
+        eng.iterate(1)  # rs_iterate records events on its launch stream around the graph replay
+    barrier()
+    s1 = eng.stats()
     wall = time.perf_counter() - wall0
     clocks = sampler.stop() if sampler else None
-    dev_ms = float(np.median(reps))
-    ms_per_step = dev_ms / steps
+    launches = int(s1.kernel_launches - s0.kernel_launches)
+    ms_per_step = max_over_ranks(s1.device_ms - s0.device_ms) / steps
     value = 1000.0 / ms_per_step
+    if dump_dir is not None:
+        write_outputs(dump_dir, collect_outputs(eng, w, tree, ranges))
 
     # ---- end to end through the C ABI with host buffers ----
     # per step: H2D of both players' range weights (the host input of a re-solve step) from pinned memory,
@@ -373,7 +429,7 @@ def measure(cx, name: str, steps: int, warmup: int, min_seconds: float, with_clo
     exploit = {"iterations": int(st_end.iterations), "chips": chips, "mbb_per_game": 1000.0 * chips / BB_CHIPS, "bb_chips": BB_CHIPS,
                "pct_of_starting_pot": 100.0 * chips / float(w.options.starting_pot), "best_response_values": [br[0], br[1]]}
     out = {"value": value, "ms_per_step": ms_per_step, "updates_per_iteration": upd_global, "updates_per_sec": value * upd_global,
-           "gpu_launches": launches * len(reps), "launches_per_step": launches / steps, "repetitions": len(reps),
+           "gpu_launches": launches, "launches_per_step": launches / steps,
            "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
                    "what": "per step: rs_set_range_weights x2 from pinned host memory, rs_iterate(1), rs_root_values x2"},
            "roofline": roofline, "exploitability": exploit, "clocks": clocks, "engine_create_s": create_s,
@@ -450,19 +506,19 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     cx.flush_l2 = flush_l2
-    steps, warmup = max(1, args.steps), max(0, args.warmup)
+    steps, warmup = args.steps, args.warmup
     if warmup < 3 and cx.rank == 0:
         print(f"bench.py: --warmup {warmup} is below the 3 warm-up steps the timing rules ask for", file=sys.stderr)
-    main = measure(cx, args.workload, steps, warmup, MIN_TIMED_SECONDS, with_clocks=True)
+    main = measure(cx, args.workload, steps, warmup, with_clocks=True, dump_dir=args.dump_outputs)
     extra = {}
     if not args.no_extra:
         for name in ("config2", "config5"):
             if name != args.workload:
-                m = measure(cx, name, 20, max(warmup, 3), 0.5, with_clocks=False)
+                m = measure(cx, name, 20, max(warmup, 3), with_clocks=False)
                 extra[name] = {"config": config_dict(name, cx.world), "value": m["value"], "unit": UNIT, "ms_per_step": m["ms_per_step"],
                                "updates_per_sec": m["updates_per_sec"], "e2e": m["e2e"],
                                "roofline": {k: m["roofline"][k] for k in ("frac", "achieved", "peak", "ms_per_launch", "algorithmic_bytes_per_launch", "whole_iteration_frac")},
-                               "exploitability": m["exploitability"], "exchange": m["exchange"], "repetitions": m["repetitions"]}
+                               "exploitability": m["exploitability"], "exchange": m["exchange"]}
     parity = None
     if cx.world > 1 and not args.no_parity:
         # the sharded path against the fp64 oracle on the live ranks: turn- and flop-rooted games, both exchange paths
@@ -499,7 +555,7 @@ def run_ours(args):
             "dtype": "f32", "data": "synthetic", "config": cfg,
             "updates_per_iteration": main["updates_per_iteration"], "updates_per_sec": main["updates_per_sec"],
             "gpu_launches": main["gpu_launches"], "launches_per_step": main["launches_per_step"],
-            "timed_region": {"repetitions": main["repetitions"], "statistic": "median repetition of K steps", "wall_s": main["wall_s_timed_region"]},
+            "timed_region": {"steps": steps, "statistic": "device time of the K steps summed", "wall_s": main["wall_s_timed_region"]},
             "e2e": main["e2e"], "roofline": main["roofline"], "cpu_baseline": cpu,
             "exploitability": main["exploitability"], "exploitability_vs_oracle": expl_check, "clocks": main["clocks"],
             "exchange": main["exchange"], "table_bytes_per_gpu": main["table_bytes_per_gpu"], "engine_create_s": main["engine_create_s"],
@@ -522,7 +578,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the config 2 / config 5 lines reported under `extra`")
     ap.add_argument("--no-parity", action="store_true", help="N > 1: skip the sharded-parity cases after the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="write the engine's outputs after the last timed step of the main workload to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs is not None and (args.gpus != 1 or args.impl != "ours"):
+        ap.error("--dump-outputs needs --gpus 1 and --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     world = int(os.environ.get("WORLD_SIZE", "1"))
