@@ -346,7 +346,7 @@ int Engine::init(const rs_config* cfg) {
             CU(R.cl_pos[q].upload(slice(L.cl_pos, lo, hi, 2 * hp)));
             CU(R.slot_of_pos[q].upload(slice(L.slot_of_pos, lo, hi, hp)));
             {
-                // four word planes per board: [board][word][pos] (see load_recs4)
+                // four word planes per board: [board][word][pos] (see stage_recs)
                 std::vector<HandRec> aos = slice(L.hrec, lo, hi, hp);
                 std::vector<HandRec> soa(aos.size());
                 const uint32_t* src = reinterpret_cast<const uint32_t*>(aos.data());

@@ -116,6 +116,8 @@ struct Ctx {
 //   SM_WSA / SM_WSB [32] warp totals of the two scans
 //   SM_B   [64]          boundaries of the opponent's non-empty card lists: B[j] = GB at the start of list j, B[J] = the
 //                        total; B[54] = B[55] = 0 for a card the opponent does not hold (tasks.h: HandRec)
+//   SM_WSC / SM_WSD [32] warp totals of the two scans of a fold reach scanned alongside (scan_reach<true>)
+//   SM_BF  [64]          the boundaries B of that fold reach
 //   SM_REC [4][HCAP]     the traverser's per-hand records of the board, staged by cp.async at the start of a task
 //   SM_CL  [HCAP] words  the opponent's per-card lists of the board (u16 pairs), staged the same way
 //   SM_X   [slots][Hx]   scratch vectors (terminal-child reach, bucketed rows), Hx known at run time
@@ -127,9 +129,12 @@ extern __shared__ __align__(16) float smem_raw[];
 #define SM_WSA (smem_raw + 4 * HCAP + 12)
 #define SM_WSB (smem_raw + 4 * HCAP + 44)
 #define SM_B (smem_raw + 4 * HCAP + 76)
-#define SM_REC (reinterpret_cast<uint32_t*>(smem_raw + 4 * HCAP + 140))
-#define SM_CL (reinterpret_cast<uint32_t*>(smem_raw + 8 * HCAP + 140))
-#define SM_X (smem_raw + 9 * HCAP + 140)
+#define SM_WSC (smem_raw + 4 * HCAP + 140)
+#define SM_WSD (smem_raw + 4 * HCAP + 172)
+#define SM_BF (smem_raw + 4 * HCAP + 204)
+#define SM_REC (reinterpret_cast<uint32_t*>(smem_raw + 4 * HCAP + 268))
+#define SM_CL (reinterpret_cast<uint32_t*>(smem_raw + 8 * HCAP + 268))
+#define SM_X (smem_raw + 9 * HCAP + 268)
 
 // Copy the thread's eight entries of the opponent's per-card lists (cl_pos of the board, u16) into shared memory with
 // cp.async; scan_reach reads them back.  Like the hand records (stage_recs) this is issued when a task starts, so the
@@ -146,11 +151,24 @@ __device__ __forceinline__ void stage_lists_raw(int tid, int HoP, const uint16_t
 //   GB[e] = reach of the first e entries of the opponent's concatenated per-card lists
 // One pass: every thread scans its 4 positions and its 8 list entries; warp shuffles + one cross-warp step.
 // Returns the total reach (all threads).
-__device__ __forceinline__ float scan_reach(const Ctx& c, const float* r) {
-    csync(c.nc);  // r is complete; previous readers of P / GB are done
+//
+// FOLD: the same pass also scans a second reach vector rf for what a fold value needs (hand_mass): its total, returned
+// in *total_f, and its list boundaries in SM_BF; it writes no P or GB.  An opponent node with a fold and a showdown child
+// values both after one pass (three barriers) instead of two.  Every sum of rf is formed exactly as a scan of rf alone
+// would form it, so the values are bit-identical either way.
+template <bool FOLD>
+__device__ __forceinline__ float scan_reach(const Ctx& c, const float* r, const float* rf = nullptr, float* total_f = nullptr) {
+    csync(c.nc);  // r (and rf) are complete; previous readers of P / GB / B are done
     float4 x = f4zero();
-    if (c.pos4 < c.HoP) x = *reinterpret_cast<const float4*>(r + c.pos4);
-    float y[8];
+    float lc = 0.f;  // FOLD: the thread's four positions of rf, summed as they are loaded
+    if (c.pos4 < c.HoP) {
+        x = *reinterpret_cast<const float4*>(r + c.pos4);
+        if (FOLD) {
+            const float4 xf = *reinterpret_cast<const float4*>(rf + c.pos4);
+            lc = (xf.x + xf.y) + (xf.z + xf.w);
+        }
+    }
+    float y[8], yf[8];
     uint32_t w[4];
     {
         // the thread's eight list entries were staged by stage_lists when the task started
@@ -166,37 +184,71 @@ __device__ __forceinline__ float scan_reach(const Ctx& c, const float* r) {
             const uint32_t a = w[i] & CL_POS_MASK, b = (w[i] >> 16) & CL_POS_MASK;
             y[2 * i] = a != CL_POS_NONE ? r[a] : 0.f;
             y[2 * i + 1] = b != CL_POS_NONE ? r[b] : 0.f;
+            if (FOLD) {
+                yf[2 * i] = a != CL_POS_NONE ? rf[a] : 0.f;
+                yf[2 * i + 1] = b != CL_POS_NONE ? rf[b] : 0.f;
+            }
         }
     }
     const float la = (x.x + x.y) + (x.z + x.w);
-    float lb = 0.f;
+    float lb = 0.f, ld = 0.f;
 #pragma unroll
-    for (int i = 0; i < 8; ++i) lb += y[i];
-    float ia = la, ib = lb;
+    for (int i = 0; i < 8; ++i) {
+        lb += y[i];
+        if (FOLD) ld += yf[i];
+    }
+    float ia = la, ib = lb, ic = lc, id = ld;
 #pragma unroll
     for (int d = 1; d < 32; d <<= 1) {
         const float ta = __shfl_up_sync(0xffffffffu, ia, d);
         const float tb = __shfl_up_sync(0xffffffffu, ib, d);
+        float tc = 0.f, td = 0.f;
+        if (FOLD) {
+            tc = __shfl_up_sync(0xffffffffu, ic, d);
+            td = __shfl_up_sync(0xffffffffu, id, d);
+        }
         if (c.lane >= d) {
             ia += ta;
             ib += tb;
+            if (FOLD) {
+                ic += tc;
+                id += td;
+            }
         }
     }
     if (c.lane == 31) {
         SM_WSA[c.warp] = ia;
         SM_WSB[c.warp] = ib;
+        if (FOLD) {
+            SM_WSC[c.warp] = ic;
+            SM_WSD[c.warp] = id;
+        }
     }
     csync(c.nc);
     // every warp scans the (<= 11) warp totals itself
     float wa = c.lane < c.nwarps ? SM_WSA[c.lane] : 0.f;
     float wb = c.lane < c.nwarps ? SM_WSB[c.lane] : 0.f;
+    float wc = 0.f, wd = 0.f;
+    if (FOLD) {
+        wc = c.lane < c.nwarps ? SM_WSC[c.lane] : 0.f;
+        wd = c.lane < c.nwarps ? SM_WSD[c.lane] : 0.f;
+    }
 #pragma unroll
     for (int d = 1; d < 16; d <<= 1) {
         const float ta = __shfl_up_sync(0xffffffffu, wa, d);
         const float tb = __shfl_up_sync(0xffffffffu, wb, d);
+        float tc = 0.f, td = 0.f;
+        if (FOLD) {
+            tc = __shfl_up_sync(0xffffffffu, wc, d);
+            td = __shfl_up_sync(0xffffffffu, wd, d);
+        }
         if (c.lane >= d) {
             wa += ta;
             wb += tb;
+            if (FOLD) {
+                wc += tc;
+                wd += td;
+            }
         }
     }
     const float total = __shfl_sync(0xffffffffu, wa, c.nwarps - 1);
@@ -204,6 +256,13 @@ __device__ __forceinline__ float scan_reach(const Ctx& c, const float* r) {
     const float base_a = c.warp > 0 ? __shfl_sync(0xffffffffu, wa, c.warp - 1) : 0.f;
     const float base_b = c.warp > 0 ? __shfl_sync(0xffffffffu, wb, c.warp - 1) : 0.f;
     float ea = base_a + ia - la, eb = base_b + ib - lb;
+    float total_d = 0.f, ed = 0.f;
+    if (FOLD) {
+        *total_f = __shfl_sync(0xffffffffu, wc, c.nwarps - 1);
+        total_d = __shfl_sync(0xffffffffu, wd, c.nwarps - 1);
+        const float base_d = c.warp > 0 ? __shfl_sync(0xffffffffu, wd, c.warp - 1) : 0.f;
+        ed = base_d + id - ld;
+    }
     if (c.pos4 < c.HoP) {
         float4 o;
         o.x = ea;
@@ -227,7 +286,8 @@ __device__ __forceinline__ float scan_reach(const Ctx& c, const float* r) {
         // boundaries of the card lists: an entry flagged CL_FIRST stores its exclusive prefix as B[ordinal]; the thread's
         // first ordinal rides in the spare bits of its first two entries (thread 0 carries the number of lists there)
         const uint32_t ord0 = ((w[0] >> 11) & 7u) | (((w[0] >> 27) & 7u) << 3);
-        float* bp = SM_B + (c.tid == 0 ? 0u : ord0);
+        const uint32_t b0 = c.tid == 0 ? 0u : ord0;
+        float* bp = SM_B + b0;
         const float ex[8] = {o0.x, o0.y, o0.z, o0.w, o1.x, o1.y, o1.z, o1.w};
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
@@ -235,6 +295,17 @@ __device__ __forceinline__ float scan_reach(const Ctx& c, const float* r) {
             if (first) *bp++ = ex[i];
         }
         if (c.tid == 0) SM_B[ord0] = total_b;  // ord0 of thread 0 = J, the number of non-empty lists
+        if (FOLD) {  // the same exclusive prefixes of rf, kept only at the list boundaries
+            float* bf = SM_BF + b0;
+            float e = ed;
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+                const bool first = ((w[i >> 1] >> ((i & 1) * 16)) & CL_FIRST) != 0;
+                if (first) *bf++ = e;
+                e += yf[i];
+            }
+            if (c.tid == 0) SM_BF[ord0] = total_d;
+        }
     }
     if (c.tid == 0) {
         SM_P[c.HoP] = total;
@@ -244,19 +315,8 @@ __device__ __forceinline__ float scan_reach(const Ctx& c, const float* r) {
     return total;
 }
 
-// The per-hand records of a board are stored as four word planes [4][Hpad]: one 128-bit load per plane gives the
+// The per-hand records of a board are stored as four word planes [4][Hpad]: one 128-bit copy per plane gives the
 // thread the same word of its four hands, fully coalesced across the warp.
-__device__ __forceinline__ void load_recs4(const uint32_t* __restrict__ planes, int HpP, int pos4, uint4 (&rec)[4]) {
-    const uint4 w0 = __ldg(reinterpret_cast<const uint4*>(planes + pos4));
-    const uint4 w1 = __ldg(reinterpret_cast<const uint4*>(planes + HpP + pos4));
-    const uint4 w2 = __ldg(reinterpret_cast<const uint4*>(planes + 2 * HpP + pos4));
-    const uint4 w3 = __ldg(reinterpret_cast<const uint4*>(planes + 3 * HpP + pos4));
-    rec[0] = make_uint4(w0.x, w1.x, w2.x, w3.x);
-    rec[1] = make_uint4(w0.y, w1.y, w2.y, w3.y);
-    rec[2] = make_uint4(w0.z, w1.z, w2.z, w3.z);
-    rec[3] = make_uint4(w0.w, w1.w, w2.w, w3.w);
-}
-
 // The records are needed only after the first scan of a task.  Loading them into registers up front would cost 16
 // registers across the scan, loading them afterwards exposes an L2 round trip: instead every thread copies its own
 // 4 x 16 bytes into shared memory with cp.async when the task starts and reads them back when it needs them (no
@@ -296,9 +356,10 @@ __device__ __forceinline__ void hand_terms(const Ctx& c, const float* r, float t
     sd = ldsb(SM_P, rec.x & 0xffffu) + ldsb(SM_P, rec.x >> 16) - total - ldsb(SM_GB, rec.y & 0xffffu) - ldsb(SM_GB, rec.y >> 16) + g0s + g0e -
          ldsb(SM_GB, rec.z & 0xffffu) - ldsb(SM_GB, rec.z >> 16) + g1s + g1e;
 }
-__device__ __forceinline__ float hand_mass(const Ctx& c, const float* r, float total, const uint4& rec) {
+// B: the boundaries of r's scan (SM_B, or SM_BF for the fold reach of scan_reach<true>)
+__device__ __forceinline__ float hand_mass(const float* B, const float* r, float total, const uint4& rec) {
     const uint32_t k0 = rec.w & 0x1ffu, k1 = (rec.w >> 9) & 0x1ffu, same4 = rec.w >> 18;
-    return total - (ldsb(SM_B + 1, k0) - ldsb(SM_B, k0)) - (ldsb(SM_B + 1, k1) - ldsb(SM_B, k1)) + (same4 != HREC_SAME_NONE ? ldsb(r, same4) : 0.f);
+    return total - (ldsb(B + 1, k0) - ldsb(B, k0)) - (ldsb(B + 1, k1) - ldsb(B, k1)) + (same4 != HREC_SAME_NONE ? ldsb(r, same4) : 0.f);
 }
 
 // Opponent reach of the thread's four positions for this task (masked by what the board removes).
@@ -422,6 +483,81 @@ __device__ __forceinline__ void xs_pick(const TaskArgs& A, float u, float (&sg)[
     for (int a = 0; a < NA; ++a) sg[a] = (a == pick) ? (A.xs_mode == 2 ? sg[a] : 1.0f) : 0.f;
 }
 
+// The terminal children of an opponent node (cfr.rs:523-558), whose reach vectors are staged in SM_X slots 0, 1, ... in
+// action order, and the hand records and per-card lists staged by cp.async.  Stores the node's terminal partial value:
+// the sum of coef * term over those children, accumulated in action order.  A fold and a showdown child (most river
+// opponent nodes) share one scan pass; any other set of terminal children is scanned child by child.
+__device__ __forceinline__ void down_terminals(const Ctx& c, const NodeTask& nt, const RoundArgs& Rk, int b, int n_act) {
+    const uint32_t nl_p = Rk.rp[c.p].n_live[b];
+    const float scale = Rk.chance_scale[b];
+    int n_fold = 0, n_sd = 0, a_fold = 0, a_sd = 0;
+    for (int a = 0; a < n_act; ++a) {
+        const int ck = nt.child[a].kind;
+        if (ck == CK_FOLD) {
+            ++n_fold;
+            a_fold = a;
+        } else if (ck == CK_SHOWDOWN) {
+            ++n_sd;
+            a_sd = a;
+        }
+    }
+    float4 acc = f4zero();
+    if (n_fold == 1 && n_sd == 1) {
+        const bool fold_first = a_fold < a_sd;
+        const float* rf = SM_X + (fold_first ? 0 : c.Hx);
+        const float* rs = SM_X + (fold_first ? c.Hx : 0);
+        float total_f;
+        const float total = scan_reach<true>(c, rs, rf, &total_f);
+        const float cf = nt.child[a_fold].coef * scale, cs = nt.child[a_sd].coef * scale;
+        const float c0 = fold_first ? cf : cs, c1 = fold_first ? cs : cf;
+        staged_recs_wait();
+        if (c.pos4 < c.HpP) {
+            uint4 rec[4];
+            staged_recs4(c, rec);
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                if (uint32_t(c.pos4 + i) < nl_p) {
+                    float m_sd, sd;  // m_sd: the showdown reach's mass, not needed
+                    hand_terms(c, rs, total, rec[i], m_sd, sd);
+                    const float m = hand_mass(SM_BF, rf, total_f, rec[i]);
+                    const float t0 = fold_first ? m : sd, t1 = fold_first ? sd : m;
+                    f4set(acc, i, f4get(acc, i) + c0 * t0);
+                    f4set(acc, i, f4get(acc, i) + c1 * t1);
+                }
+            }
+        }
+    } else {
+        int slot = 0;
+        for (int a = 0; a < n_act; ++a) {
+            const int ck = nt.child[a].kind;
+            if (ck != CK_FOLD && ck != CK_SHOWDOWN) continue;
+            const float* r = SM_X + slot * c.Hx;
+            ++slot;
+            const float cf = nt.child[a].coef * scale;
+            const float total = scan_reach<false>(c, r);
+            staged_recs_wait();
+            if (c.pos4 < c.HpP) {
+                uint4 rec[4];
+                staged_recs4(c, rec);  // read back for every terminal child instead of held in registers across the scans
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                    if (uint32_t(c.pos4 + i) < nl_p) {
+                        float m, sd;
+                        if (ck == CK_FOLD) {
+                            m = hand_mass(SM_B, r, total, rec[i]);
+                            f4set(acc, i, f4get(acc, i) + cf * m);
+                        } else {
+                            hand_terms(c, r, total, rec[i], m, sd);
+                            f4set(acc, i, f4get(acc, i) + cf * sd);
+                        }
+                    }
+                }
+            }
+        }
+    }
+    if (c.pos4 < c.HpP) stcg4(Rk.cbuf + (size_t(nt.out) * Rk.n_boards + b) * c.HpP + c.pos4, acc);
+}
+
 template <int MODE, int NA, bool XS>
 __device__ __forceinline__ void task_down(const TaskArgs& A, const Ctx& c, const NodeTask& nt, const RoundArgs& Rk, int k, int b) {
     const DevRoundPlayer& O = Rk.rp[c.o];
@@ -459,39 +595,7 @@ __device__ __forceinline__ void task_down(const TaskArgs& A, const Ctx& c, const
         if (ck == CK_FOLD || ck == CK_SHOWDOWN) ++slot;
     }
     if (nt.out < 0) return;
-    // terminal children: their values only depend on the child reach staged in shared memory
-    const DevRoundPlayer& Pp = Rk.rp[c.p];
-    const uint32_t nl_p = Pp.n_live[b];
-    const float scale = Rk.chance_scale[b];
-    float4 acc = f4zero();
-    slot = 0;
-    for (int a = 0; a < NA; ++a) {
-        const int ck = nt.child[a].kind;
-        if (ck != CK_FOLD && ck != CK_SHOWDOWN) continue;
-        const float* r = SM_X + slot * c.Hx;
-        ++slot;
-        const float cf = nt.child[a].coef * scale;
-        const float total = scan_reach(c, r);
-        staged_recs_wait();
-        if (c.pos4 < c.HpP) {
-            uint4 rec[4];
-            staged_recs4(c, rec);  // read back for every terminal child instead of held in registers across the scans
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                if (uint32_t(c.pos4 + i) < nl_p) {
-                    float m, sd;
-                    if (ck == CK_FOLD) {
-                        m = hand_mass(c, r, total, rec[i]);
-                        f4set(acc, i, f4get(acc, i) + cf * m);
-                    } else {
-                        hand_terms(c, r, total, rec[i], m, sd);
-                        f4set(acc, i, f4get(acc, i) + cf * sd);
-                    }
-                }
-            }
-        }
-    }
-    if (c.pos4 < c.HpP) stcg4(Rk.cbuf + (size_t(nt.out) * Rk.n_boards + b) * c.HpP + c.pos4, acc);
+    down_terminals(c, nt, Rk, b, NA);
 }
 
 // any number of actions, any row mapping: scalar loads, two passes over the actions
@@ -537,33 +641,10 @@ __device__ __forceinline__ void task_down_generic(const TaskArgs& A, const Ctx& 
         }
     }
     if (nt.out < 0) return;
-    const DevRoundPlayer& Pp = Rk.rp[c.p];
-    const uint32_t nl_p = Pp.n_live[b];
-    const float scale = Rk.chance_scale[b];
-    stage_lists_raw(c.tid, c.HoP, O.cl_pos + size_t(b) * 2 * c.HoP);  // generic path: staged right before the scans
-    float4 acc = f4zero();
-    uint4 rec[4];
-    if (c.pos4 < c.HpP) load_recs4(reinterpret_cast<const uint32_t*>(Pp.hrec) + size_t(b) * 4 * c.HpP, c.HpP, c.pos4, rec);
-    int slot = 0;
-    for (int a = 0; a < n_act; ++a) {
-        const int ck = nt.child[a].kind;
-        if (ck != CK_FOLD && ck != CK_SHOWDOWN) continue;
-        const float* r = SM_X + slot * c.Hx;
-        ++slot;
-        const float cf = nt.child[a].coef * scale;
-        const float total = scan_reach(c, r);
-        if (c.pos4 < c.HpP) {
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                if (uint32_t(c.pos4 + i) < nl_p) {
-                    float m, sd;
-                    hand_terms(c, r, total, rec[i], m, sd);
-                    f4set(acc, i, f4get(acc, i) + cf * (ck == CK_FOLD ? m : sd));
-                }
-            }
-        }
-    }
-    if (c.pos4 < c.HpP) stcg4(Rk.cbuf + (size_t(nt.out) * Rk.n_boards + b) * c.HpP + c.pos4, acc);
+    // generic path: staged right before the scans
+    stage_lists_raw(c.tid, c.HoP, O.cl_pos + size_t(b) * 2 * c.HoP);
+    stage_recs(c, reinterpret_cast<const uint32_t*>(Rk.rp[c.p].hrec) + size_t(b) * 4 * c.HpP);
+    down_terminals(c, nt, Rk, b, n_act);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -577,7 +658,7 @@ __device__ __forceinline__ void trav_terms(const TaskArgs& A, const Ctx& c, cons
     stage_recs(c, reinterpret_cast<const uint32_t*>(Pp.hrec) + size_t(b) * 4 * c.HpP);
     const float4 r4 = load_reach4(A, c, nt, Rk, k, b);
     if (c.pos4 < c.HoP) *reinterpret_cast<float4*>(SM_RS + c.pos4) = r4;
-    const float total = scan_reach(c, SM_RS);
+    const float total = scan_reach<false>(c, SM_RS);
     mass = f4zero();
     sd = f4zero();
     const uint32_t nl_p = Pp.n_live[b];
@@ -590,7 +671,7 @@ __device__ __forceinline__ void trav_terms(const TaskArgs& A, const Ctx& c, cons
             if (uint32_t(c.pos4 + i) < nl_p) {
                 float m, s = 0.f;
                 if (need_sd) hand_terms(c, SM_RS, total, rec[i], m, s);
-                else m = hand_mass(c, SM_RS, total, rec[i]);
+                else m = hand_mass(SM_B, SM_RS, total, rec[i]);
                 f4set(mass, i, m);
                 f4set(sd, i, s);
             }
@@ -870,7 +951,7 @@ __global__ void __launch_bounds__(MAXT + 32, MINB) task_kernel(const __grid_cons
     const int NC = blockDim.x - 32;  // compute threads; the last warp is the dispatcher
     const int tid = threadIdx.x;
     if (tid == 0) mbar_init(&s_done, uint32_t(NC >> 5));
-    if (tid < 2) SM_B[54 + tid] = 0.f;  // boundaries of "a card the opponent does not hold" (HREC_K_NONE), never overwritten
+    if (tid < 2) SM_B[54 + tid] = SM_BF[54 + tid] = 0.f;  // boundaries of "a card the opponent does not hold" (HREC_K_NONE), never overwritten
     __syncthreads();
 
     if (tid >= NC) {
@@ -1234,7 +1315,7 @@ __global__ void unpermute_kernel(const float* __restrict__ in, const uint16_t* _
 
 size_t task_kernel_smem_bytes(int slots, int Hp_pad, int Ho_pad) {
     const int hx = Hp_pad > Ho_pad ? Hp_pad : Ho_pad;
-    size_t floats = size_t(9 * HCAP + 140) + size_t(slots) * hx;  // fixed-offset arrays (SM_*), then the scratch vectors
+    size_t floats = size_t(9 * HCAP + 268) + size_t(slots) * hx;  // fixed-offset arrays (SM_*), then the scratch vectors
     return floats * sizeof(float);
 }
 
