@@ -217,7 +217,8 @@ struct Engine {
     size_t st_stride = 0, st_smem = 0;
     int st_XP = 0, st_rows = 0, st_vy_rows = 0, st_vm_rows = 0, st_slots = 0, st_threads = 0, st_blocks_per_sm = 1, st_qs = 1, st_qm = 1;
     int slots = 1;
-    size_t smem_bytes = 0;
+    size_t smem_bytes = 0;  // dynamic shared memory of the wide task-kernel build
+    size_t smem_small = 0;  // of the 288-thread build
     int blocks_per_sm = 1, n_sms = 148;
     int round_threads[3] = {0, 0, 0};  // compute threads the tasks of round k need: live hands / 4, a warp multiple
     int bps_small = 0;                 // resident CTAs per SM of the 288-thread specialisation (0: no round fits it)
@@ -416,7 +417,7 @@ int Engine::init(const rs_config* cfg) {
         *abort_host = 0;
         CU(cudaHostGetDevicePointer(reinterpret_cast<void**>(&abort_dev), abort_host, 0));
     }
-    size_t smem_need = std::max(task_kernel_smem_bytes(slots, HP[0], HP[1]), task_kernel_smem_bytes(slots, HP[1], HP[0]));
+    size_t smem_need = std::max(task_kernel_smem_bytes(true, slots, HP[0], HP[1]), task_kernel_smem_bytes(true, slots, HP[1], HP[0]));
     int max_optin = 0;
     CU(cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
     if (smem_need > size_t(max_optin))
@@ -427,7 +428,8 @@ int Engine::init(const rs_config* cfg) {
     if (blocks_per_sm < 1) return set_err(RS_ERR_UNSUPPORTED, "task kernel does not fit on an SM");
     for (uint32_t k = 0; k < P.n_rounds; ++k)
         if (round_threads[k] <= 288 && bps_small == 0) {
-            CU(configure_task_kernels(smem_need, 288, false, &bps_small));
+            smem_small = std::max(task_kernel_smem_bytes(false, slots, HP[0], HP[1]), task_kernel_smem_bytes(false, slots, HP[1], HP[0]));
+            CU(configure_task_kernels(smem_small, 288, false, &bps_small));
             if (bps_small < 1) return set_err(RS_ERR_UNSUPPORTED, "task kernel does not fit on an SM");
         }
     n_sms = prop.multiProcessorCount;
@@ -826,7 +828,7 @@ int Engine::enqueue_traversal(int trav, int mode, uint64_t* count, const TaskSet
                 const int thr = pieces[i].threads;
                 const bool wide = wide_for(thr, a.t1 - a.t0);
                 const int grid = int(std::min<uint64_t>(uint64_t(a.t1 - a.t0), uint64_t(n_sms) * (wide ? blocks_per_sm : bps_small)));
-                CU(launch_task_kernel(a, mode, grid, thr, wide, smem_bytes, stream));
+                CU(launch_task_kernel(a, mode, grid, thr, wide, wide ? smem_bytes : smem_small, stream));
                 uint64_t bytes = 0;
                 for (const TaskSet::Section& sc : set->sections)
                     if (sc.first >= a.t0 && sc.first < a.t1) {

@@ -108,37 +108,40 @@ struct Ctx {
     int p, o, Hp, Ho, HpP, HoP, Hx;
 };
 
-// Shared memory of a CTA at COMPILE-TIME offsets (capacity = the largest range, 1326 hands padded to a warp multiple of
-// four-hand threads): the arrays need no pointer registers and every access is base + immediate.
-//   SM_RS  [HCAP]        opponent reach being scanned
-//   SM_P   [HCAP + 4]    exclusive prefix of reach by position (strength order on the river)
-//   SM_GB  [2*HCAP + 8]  exclusive prefix of reach over the opponent's per-card lists
+// Shared memory of a CTA at COMPILE-TIME offsets: the arrays need no pointer registers and every access is base +
+// immediate.  The capacity HC = 4 * MAXT is what the build's threads cover (1152 positions in the 288-thread build, 1408 =
+// 1326 hands padded in the wide one): every function that touches these arrays is a template on HC.  A smaller
+// footprint leaves more of the SM's combined L1 / shared-memory array to L1 (spills, table loads).
+//   SM_RS  [HC]          opponent reach being scanned
+//   SM_P   [HC + 4]      exclusive prefix of reach by position (strength order on the river)
+//   SM_GB  [2*HC + 8]    exclusive prefix of reach over the opponent's per-card lists
 //   SM_WSA / SM_WSB [32] warp totals of the two scans
 //   SM_B   [64]          boundaries of the opponent's non-empty card lists: B[j] = GB at the start of list j, B[J] = the
 //                        total; B[54] = B[55] = 0 for a card the opponent does not hold (tasks.h: HandRec)
 //   SM_WSC / SM_WSD [32] warp totals of the two scans of a fold reach scanned alongside (scan_reach<true>)
 //   SM_BF  [64]          the boundaries B of that fold reach
-//   SM_REC [4][HCAP]     the traverser's per-hand records of the board, staged by cp.async at the start of a task
-//   SM_CL  [HCAP] words  the opponent's per-card lists of the board (u16 pairs), staged the same way
+//   SM_REC [4][HC]       the traverser's per-hand records of the board, staged by cp.async at the start of a task
+//   SM_CL  [HC] words    the opponent's per-card lists of the board (u16 pairs), staged the same way
 //   SM_X   [slots][Hx]   scratch vectors (terminal-child reach, bucketed rows), Hx known at run time
-constexpr int HCAP = MAX_TASK_THREADS * 4;
 extern __shared__ __align__(16) float smem_raw[];
 #define SM_RS (smem_raw)
-#define SM_P (smem_raw + HCAP)
-#define SM_GB (smem_raw + 2 * HCAP + 4)
-#define SM_WSA (smem_raw + 4 * HCAP + 12)
-#define SM_WSB (smem_raw + 4 * HCAP + 44)
-#define SM_B (smem_raw + 4 * HCAP + 76)
-#define SM_WSC (smem_raw + 4 * HCAP + 140)
-#define SM_WSD (smem_raw + 4 * HCAP + 172)
-#define SM_BF (smem_raw + 4 * HCAP + 204)
-#define SM_REC (reinterpret_cast<uint32_t*>(smem_raw + 4 * HCAP + 268))
-#define SM_CL (reinterpret_cast<uint32_t*>(smem_raw + 8 * HCAP + 268))
-#define SM_X (smem_raw + 9 * HCAP + 268)
+#define SM_P (smem_raw + HC)
+#define SM_GB (smem_raw + 2 * HC + 4)
+#define SM_WSA (smem_raw + 4 * HC + 12)
+#define SM_WSB (smem_raw + 4 * HC + 44)
+#define SM_B (smem_raw + 4 * HC + 76)
+#define SM_WSC (smem_raw + 4 * HC + 140)
+#define SM_WSD (smem_raw + 4 * HC + 172)
+#define SM_BF (smem_raw + 4 * HC + 204)
+#define SM_REC (reinterpret_cast<uint32_t*>(smem_raw + 4 * HC + 268))
+#define SM_CL (reinterpret_cast<uint32_t*>(smem_raw + 8 * HC + 268))
+#define SM_X (smem_raw + 9 * HC + 268)
+constexpr int smem_fixed_floats(int HC) { return 9 * HC + 268; }
 
 // Copy the thread's eight entries of the opponent's per-card lists (cl_pos of the board, u16) into shared memory with
 // cp.async; scan_reach reads them back.  Like the hand records (stage_recs) this is issued when a task starts, so the
 // L2 round trip overlaps the reach load instead of following it, and costs no registers.
+template <int HC>
 __device__ __forceinline__ void stage_lists_raw(int tid, int HoP, const uint16_t* __restrict__ cl_pos_b) {
     if (8 * tid < 2 * HoP)
         asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(uint32_t(__cvta_generic_to_shared(SM_CL + 4 * tid))), "l"(cl_pos_b + 8 * tid)
@@ -150,15 +153,18 @@ __device__ __forceinline__ void stage_lists_raw(int tid, int HoP, const uint16_t
 //   P[i]  = reach of the i weakest hands           (position order)
 //   GB[e] = reach of the first e entries of the opponent's concatenated per-card lists
 // One pass: every thread scans its 4 positions and its 8 list entries; warp shuffles + one cross-warp step.
-// Returns the total reach (all threads).
+// Returns the total reach (all threads).  Positions from 4 * nc on are not scanned (a round launched with fewer threads
+// holds no live hand there), so in the 288-thread build, whose arrays end at 4 * 288 positions, the totals go to
+// P[min(HoP, 4 * nc)] and GB[2 * min(HoP, 4 * nc)].
 //
 // FOLD: the same pass also scans a second reach vector rf for what a fold value needs (hand_mass): its total, returned
 // in *total_f, and its list boundaries in SM_BF; it writes no P or GB.  An opponent node with a fold and a showdown child
 // values both after one pass (three barriers) instead of two.  Every sum of rf is formed exactly as a scan of rf alone
 // would form it, so the values are bit-identical either way.
-template <bool FOLD>
+template <int HC, bool FOLD>
 __device__ __forceinline__ float scan_reach(const Ctx& c, const float* r, const float* rf = nullptr, float* total_f = nullptr) {
     csync(c.nc);  // r (and rf) are complete; previous readers of P / GB / B are done
+    const int hend = HC >= 4 * MAX_TASK_THREADS ? c.HoP : min(c.HoP, 4 * c.nc);  // the wide build holds every HoP
     float4 x = f4zero();
     float lc = 0.f;  // FOLD: the thread's four positions of rf, summed as they are loaded
     if (c.pos4 < c.HoP) {
@@ -308,8 +314,8 @@ __device__ __forceinline__ float scan_reach(const Ctx& c, const float* r, const 
         }
     }
     if (c.tid == 0) {
-        SM_P[c.HoP] = total;
-        SM_GB[2 * c.HoP] = total_b;
+        SM_P[hend] = total;
+        SM_GB[2 * hend] = total_b;
     }
     csync(c.nc);
     return total;
@@ -321,22 +327,24 @@ __device__ __forceinline__ float scan_reach(const Ctx& c, const float* r, const 
 // registers across the scan, loading them afterwards exposes an L2 round trip: instead every thread copies its own
 // 4 x 16 bytes into shared memory with cp.async when the task starts and reads them back when it needs them (no
 // barrier: a thread only ever reads what it copied itself).
+template <int HC>
 __device__ __forceinline__ void stage_recs(const Ctx& c, const uint32_t* __restrict__ planes) {
     if (c.pos4 < c.HpP) {
 #pragma unroll
         for (int w = 0; w < 4; ++w)
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(uint32_t(__cvta_generic_to_shared(SM_REC + w * HCAP + c.pos4))),
+            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(uint32_t(__cvta_generic_to_shared(SM_REC + w * HC + c.pos4))),
                          "l"(planes + size_t(w) * c.HpP + c.pos4)
                          : "memory");
     }
     asm volatile("cp.async.commit_group;" ::: "memory");
 }
 __device__ __forceinline__ void staged_recs_wait() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
+template <int HC>
 __device__ __forceinline__ void staged_recs4(const Ctx& c, uint4 (&rec)[4]) {
     const uint4 w0 = *reinterpret_cast<const uint4*>(SM_REC + c.pos4);
-    const uint4 w1 = *reinterpret_cast<const uint4*>(SM_REC + HCAP + c.pos4);
-    const uint4 w2 = *reinterpret_cast<const uint4*>(SM_REC + 2 * HCAP + c.pos4);
-    const uint4 w3 = *reinterpret_cast<const uint4*>(SM_REC + 3 * HCAP + c.pos4);
+    const uint4 w1 = *reinterpret_cast<const uint4*>(SM_REC + HC + c.pos4);
+    const uint4 w2 = *reinterpret_cast<const uint4*>(SM_REC + 2 * HC + c.pos4);
+    const uint4 w3 = *reinterpret_cast<const uint4*>(SM_REC + 3 * HC + c.pos4);
     rec[0] = make_uint4(w0.x, w1.x, w2.x, w3.x);
     rec[1] = make_uint4(w0.y, w1.y, w2.y, w3.y);
     rec[2] = make_uint4(w0.z, w1.z, w2.z, w3.z);
@@ -349,6 +357,7 @@ __device__ __forceinline__ void staged_recs4(const Ctx& c, uint4 (&rec)[4]) {
 __device__ __forceinline__ float ldsb(const float* base, uint32_t byte_off) {  // shared-memory load at base + byte offset
     return *reinterpret_cast<const float*>(reinterpret_cast<const char*>(base) + byte_off);
 }
+template <int HC>
 __device__ __forceinline__ void hand_terms(const Ctx& c, const float* r, float total, const uint4& rec, float& mass, float& sd) {
     const uint32_t k0 = rec.w & 0x1ffu, k1 = (rec.w >> 9) & 0x1ffu, same4 = rec.w >> 18;
     const float g0s = ldsb(SM_B, k0), g0e = ldsb(SM_B + 1, k0), g1s = ldsb(SM_B, k1), g1e = ldsb(SM_B + 1, k1);
@@ -487,6 +496,7 @@ __device__ __forceinline__ void xs_pick(const TaskArgs& A, float u, float (&sg)[
 // action order, and the hand records and per-card lists staged by cp.async.  Stores the node's terminal partial value:
 // the sum of coef * term over those children, accumulated in action order.  A fold and a showdown child (most river
 // opponent nodes) share one scan pass; any other set of terminal children is scanned child by child.
+template <int HC>
 __device__ __forceinline__ void down_terminals(const Ctx& c, const NodeTask& nt, const RoundArgs& Rk, int b, int n_act) {
     const uint32_t nl_p = Rk.rp[c.p].n_live[b];
     const float scale = Rk.chance_scale[b];
@@ -507,18 +517,18 @@ __device__ __forceinline__ void down_terminals(const Ctx& c, const NodeTask& nt,
         const float* rf = SM_X + (fold_first ? 0 : c.Hx);
         const float* rs = SM_X + (fold_first ? c.Hx : 0);
         float total_f;
-        const float total = scan_reach<true>(c, rs, rf, &total_f);
+        const float total = scan_reach<HC, true>(c, rs, rf, &total_f);
         const float cf = nt.child[a_fold].coef * scale, cs = nt.child[a_sd].coef * scale;
         const float c0 = fold_first ? cf : cs, c1 = fold_first ? cs : cf;
         staged_recs_wait();
         if (c.pos4 < c.HpP) {
             uint4 rec[4];
-            staged_recs4(c, rec);
+            staged_recs4<HC>(c, rec);
 #pragma unroll
             for (int i = 0; i < 4; ++i) {
                 if (uint32_t(c.pos4 + i) < nl_p) {
                     float m_sd, sd;  // m_sd: the showdown reach's mass, not needed
-                    hand_terms(c, rs, total, rec[i], m_sd, sd);
+                    hand_terms<HC>(c, rs, total, rec[i], m_sd, sd);
                     const float m = hand_mass(SM_BF, rf, total_f, rec[i]);
                     const float t0 = fold_first ? m : sd, t1 = fold_first ? sd : m;
                     f4set(acc, i, f4get(acc, i) + c0 * t0);
@@ -534,11 +544,11 @@ __device__ __forceinline__ void down_terminals(const Ctx& c, const NodeTask& nt,
             const float* r = SM_X + slot * c.Hx;
             ++slot;
             const float cf = nt.child[a].coef * scale;
-            const float total = scan_reach<false>(c, r);
+            const float total = scan_reach<HC, false>(c, r);
             staged_recs_wait();
             if (c.pos4 < c.HpP) {
                 uint4 rec[4];
-                staged_recs4(c, rec);  // read back for every terminal child instead of held in registers across the scans
+                staged_recs4<HC>(c, rec);  // read back for every terminal child instead of held in registers across the scans
 #pragma unroll
                 for (int i = 0; i < 4; ++i) {
                     if (uint32_t(c.pos4 + i) < nl_p) {
@@ -547,7 +557,7 @@ __device__ __forceinline__ void down_terminals(const Ctx& c, const NodeTask& nt,
                             m = hand_mass(SM_B, r, total, rec[i]);
                             f4set(acc, i, f4get(acc, i) + cf * m);
                         } else {
-                            hand_terms(c, r, total, rec[i], m, sd);
+                            hand_terms<HC>(c, r, total, rec[i], m, sd);
                             f4set(acc, i, f4get(acc, i) + cf * sd);
                         }
                     }
@@ -558,14 +568,14 @@ __device__ __forceinline__ void down_terminals(const Ctx& c, const NodeTask& nt,
     if (c.pos4 < c.HpP) stcg4(Rk.cbuf + (size_t(nt.out) * Rk.n_boards + b) * c.HpP + c.pos4, acc);
 }
 
-template <int MODE, int NA, bool XS>
+template <int HC, int MODE, int NA, bool XS>
 __device__ __forceinline__ void task_down(const TaskArgs& A, const Ctx& c, const NodeTask& nt, const RoundArgs& Rk, int k, int b) {
     const DevRoundPlayer& O = Rk.rp[c.o];
     const uint32_t nrp = O.n_rows_pad[b];
     const float* __restrict__ slab = (MODE == KM_CFR ? O.regrets : O.ssum) + O.board_off[b] + size_t(nrp) * nt.cum_a;
     if (nt.out >= 0) {
-        stage_lists_raw(c.tid, c.HoP, O.cl_pos + size_t(b) * 2 * c.HoP);
-        stage_recs(c, reinterpret_cast<const uint32_t*>(Rk.rp[c.p].hrec) + size_t(b) * 4 * c.HpP);
+        stage_lists_raw<HC>(c.tid, c.HoP, O.cl_pos + size_t(b) * 2 * c.HoP);
+        stage_recs<HC>(c, reinterpret_cast<const uint32_t*>(Rk.rp[c.p].hrec) + size_t(b) * 4 * c.HpP);
     }
     const float4 r4 = load_reach4(A, c, nt, Rk, k, b);
     uint32_t rows[4] = {0xffffu, 0xffffu, 0xffffu, 0xffffu};
@@ -595,11 +605,11 @@ __device__ __forceinline__ void task_down(const TaskArgs& A, const Ctx& c, const
         if (ck == CK_FOLD || ck == CK_SHOWDOWN) ++slot;
     }
     if (nt.out < 0) return;
-    down_terminals(c, nt, Rk, b, NA);
+    down_terminals<HC>(c, nt, Rk, b, NA);
 }
 
 // any number of actions, any row mapping: scalar loads, two passes over the actions
-template <int MODE, bool XS>
+template <int HC, int MODE, bool XS>
 __device__ __forceinline__ void task_down_generic(const TaskArgs& A, const Ctx& c, const NodeTask& nt, const RoundArgs& Rk, int k, int b) {
     const DevRoundPlayer& O = Rk.rp[c.o];
     const uint32_t nrp = O.n_rows_pad[b];
@@ -642,35 +652,36 @@ __device__ __forceinline__ void task_down_generic(const TaskArgs& A, const Ctx& 
     }
     if (nt.out < 0) return;
     // generic path: staged right before the scans
-    stage_lists_raw(c.tid, c.HoP, O.cl_pos + size_t(b) * 2 * c.HoP);
-    stage_recs(c, reinterpret_cast<const uint32_t*>(Rk.rp[c.p].hrec) + size_t(b) * 4 * c.HpP);
-    down_terminals(c, nt, Rk, b, n_act);
+    stage_lists_raw<HC>(c.tid, c.HoP, O.cl_pos + size_t(b) * 2 * c.HoP);
+    stage_recs<HC>(c, reinterpret_cast<const uint32_t*>(Rk.rp[c.p].hrec) + size_t(b) * 4 * c.HpP);
+    down_terminals<HC>(c, nt, Rk, b, n_act);
 }
 
 // ------------------------------------------------------------------------------------------------
 // TK_UP_TRAV: traverser node (cfr.rs:588, 612-621)
 // ------------------------------------------------------------------------------------------------
 // common front part: stage the reach, run the scan, produce per-hand mass and showdown term
+template <int HC>
 __device__ __forceinline__ void trav_terms(const TaskArgs& A, const Ctx& c, const NodeTask& nt, const RoundArgs& Rk, int k, int b,
                                            bool need_sd, float4& mass, float4& sd) {
     const DevRoundPlayer& Pp = Rk.rp[c.p];
-    stage_lists_raw(c.tid, c.HoP, Rk.rp[c.o].cl_pos + size_t(b) * 2 * c.HoP);
-    stage_recs(c, reinterpret_cast<const uint32_t*>(Pp.hrec) + size_t(b) * 4 * c.HpP);
+    stage_lists_raw<HC>(c.tid, c.HoP, Rk.rp[c.o].cl_pos + size_t(b) * 2 * c.HoP);
+    stage_recs<HC>(c, reinterpret_cast<const uint32_t*>(Pp.hrec) + size_t(b) * 4 * c.HpP);
     const float4 r4 = load_reach4(A, c, nt, Rk, k, b);
     if (c.pos4 < c.HoP) *reinterpret_cast<float4*>(SM_RS + c.pos4) = r4;
-    const float total = scan_reach<false>(c, SM_RS);
+    const float total = scan_reach<HC, false>(c, SM_RS);
     mass = f4zero();
     sd = f4zero();
     const uint32_t nl_p = Pp.n_live[b];
     staged_recs_wait();
     if (c.pos4 < c.HpP) {
         uint4 rec[4];
-        staged_recs4(c, rec);
+        staged_recs4<HC>(c, rec);
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
             if (uint32_t(c.pos4 + i) < nl_p) {
                 float m, s = 0.f;
-                if (need_sd) hand_terms(c, SM_RS, total, rec[i], m, s);
+                if (need_sd) hand_terms<HC>(c, SM_RS, total, rec[i], m, s);
                 else m = hand_mass(SM_B, SM_RS, total, rec[i]);
                 f4set(mass, i, m);
                 f4set(sd, i, s);
@@ -681,10 +692,11 @@ __device__ __forceinline__ void trav_terms(const TaskArgs& A, const Ctx& c, cons
 
 // mass / showdown terms of a traverser node: computed here (scan + per-hand terms), or, on chain rounds, read from the
 // two value buffers the node's TK_TRAV_TERMS task left
+template <int HC>
 __device__ __forceinline__ void trav_terms_or_load(const TaskArgs& A, const Ctx& c, const NodeTask& nt, const RoundArgs& Rk, int k, int b,
                                                    bool need_sd, float4& mass, float4& sd) {
     if (!nt.pre_terms) {
-        trav_terms(A, c, nt, Rk, k, b, need_sd, mass, sd);
+        trav_terms<HC>(A, c, nt, Rk, k, b, need_sd, mass, sd);
         return;
     }
     mass = f4zero();
@@ -696,7 +708,7 @@ __device__ __forceinline__ void trav_terms_or_load(const TaskArgs& A, const Ctx&
     }
 }
 
-template <int MODE, int NA>
+template <int HC, int MODE, int NA>
 __device__ __forceinline__ void task_trav(const TaskArgs& A, const Ctx& c, const NodeTask& nt, const RoundArgs& Rk, int k, int b) {
     const DevRoundPlayer& Pp = Rk.rp[c.p];
     const float scale = Rk.chance_scale[b];
@@ -708,7 +720,7 @@ __device__ __forceinline__ void task_trav(const TaskArgs& A, const Ctx& c, const
         need_sd |= (nt.child[a].kind == CK_SHOWDOWN);
     }
     float4 mass, sd;
-    trav_terms_or_load(A, c, nt, Rk, k, b, need_sd, mass, sd);
+    trav_terms_or_load<HC>(A, c, nt, Rk, k, b, need_sd, mass, sd);
     // child values that come from other tasks: loaded after the scan (held across it they cost registers the
     // 64-register build does not have: measured +2 %)
 #pragma unroll
@@ -831,7 +843,7 @@ __device__ __forceinline__ void task_trav(const TaskArgs& A, const Ctx& c, const
 }
 
 // wide nodes (more than FAST_ACTIONS actions): values in shared memory, dynamic loops over the actions
-template <int MODE>
+template <int HC, int MODE>
 __device__ __forceinline__ void task_trav_generic(const TaskArgs& A, const Ctx& c, const NodeTask& nt, const RoundArgs& Rk, int k, int b) {
     const DevRoundPlayer& Pp = Rk.rp[c.p];
     const float scale = Rk.chance_scale[b];
@@ -843,7 +855,7 @@ __device__ __forceinline__ void task_trav_generic(const TaskArgs& A, const Ctx& 
         need_sd |= (ck == CK_SHOWDOWN);
     }
     float4 mass, sd;
-    trav_terms_or_load(A, c, nt, Rk, k, b, need_sd, mass, sd);
+    trav_terms_or_load<HC>(A, c, nt, Rk, k, b, need_sd, mass, sd);
     float* out = (nt.root_scatter ? Rk.sbuf : Rk.cbuf) + (size_t(nt.out) * Rk.n_boards + b) * c.HpP;
     if (c.pos4 < c.HpP) {
         *reinterpret_cast<float4*>(SM_X + c.pos4) = mass;
@@ -944,6 +956,7 @@ struct TaskSlot {
 
 template <int MODE, int MAXT, int MINB, bool XS>
 __global__ void __launch_bounds__(MAXT + 32, MINB) task_kernel(const __grid_constant__ TaskArgs A) {
+    constexpr int HC = 4 * MAXT;  // positions the shared-memory arrays hold
     __shared__ __align__(16) TaskSlot s_slot[2];
 
     __shared__ __align__(8) uint64_t s_done;  // phase i completes when every compute warp has finished task i
@@ -1138,21 +1151,21 @@ __global__ void __launch_bounds__(MAXT + 32, MINB) task_kernel(const __grid_cons
         switch (kind) {
             case TK_DOWN: {
                 switch (nt.n_act) {
-                    case 2: task_down<MODE, 2, XS>(A, c, nt, Rk, k, b); break;
-                    case 3: task_down<MODE, 3, XS>(A, c, nt, Rk, k, b); break;
-                    case 4: task_down<MODE, 4, XS>(A, c, nt, Rk, k, b); break;
-                    case 5: task_down<MODE, 5, XS>(A, c, nt, Rk, k, b); break;
-                    default: task_down_generic<MODE, XS>(A, c, nt, Rk, k, b); break;
+                    case 2: task_down<HC, MODE, 2, XS>(A, c, nt, Rk, k, b); break;
+                    case 3: task_down<HC, MODE, 3, XS>(A, c, nt, Rk, k, b); break;
+                    case 4: task_down<HC, MODE, 4, XS>(A, c, nt, Rk, k, b); break;
+                    case 5: task_down<HC, MODE, 5, XS>(A, c, nt, Rk, k, b); break;
+                    default: task_down_generic<HC, MODE, XS>(A, c, nt, Rk, k, b); break;
                 }
                 break;
             }
             case TK_UP_TRAV: {
                 switch (nt.n_act) {
-                    case 2: task_trav<MODE, 2>(A, c, nt, Rk, k, b); break;
-                    case 3: task_trav<MODE, 3>(A, c, nt, Rk, k, b); break;
-                    case 4: task_trav<MODE, 4>(A, c, nt, Rk, k, b); break;
-                    case 5: task_trav<MODE, 5>(A, c, nt, Rk, k, b); break;
-                    default: task_trav_generic<MODE>(A, c, nt, Rk, k, b); break;
+                    case 2: task_trav<HC, MODE, 2>(A, c, nt, Rk, k, b); break;
+                    case 3: task_trav<HC, MODE, 3>(A, c, nt, Rk, k, b); break;
+                    case 4: task_trav<HC, MODE, 4>(A, c, nt, Rk, k, b); break;
+                    case 5: task_trav<HC, MODE, 5>(A, c, nt, Rk, k, b); break;
+                    default: task_trav_generic<HC, MODE>(A, c, nt, Rk, k, b); break;
                 }
                 break;
             }
@@ -1235,7 +1248,7 @@ __global__ void __launch_bounds__(MAXT + 32, MINB) task_kernel(const __grid_cons
                 bool need_sd = false;
                 for (int a = 0; a < nt.n_act; ++a) need_sd |= (nt.child[a].kind == CK_SHOWDOWN);
                 float4 mass, sd;
-                trav_terms(A, c, nt, Rk, k, b, need_sd, mass, sd);
+                trav_terms<HC>(A, c, nt, Rk, k, b, need_sd, mass, sd);
                 if (c.pos4 < c.HpP) {
                     float* m = Rk.cbuf + (size_t(nt.out) * Rk.n_boards + b) * c.HpP + c.pos4;
                     stcg4(m, mass);
@@ -1245,7 +1258,7 @@ __global__ void __launch_bounds__(MAXT + 32, MINB) task_kernel(const __grid_cons
             }
             case TK_ROOT_SHOWDOWN: {
                 float4 mass, sd;
-                trav_terms(A, c, nt, Rk, k, b, true, mass, sd);
+                trav_terms<HC>(A, c, nt, Rk, k, b, true, mass, sd);
                 const float cf = nt.child[0].coef * Rk.chance_scale[b];
                 if (c.pos4 < c.HpP)
                     store_value4(c, nt, Rk, b, (nt.root_scatter ? Rk.sbuf : Rk.cbuf) + (size_t(nt.out) * Rk.n_boards + b) * c.HpP,
@@ -1313,9 +1326,10 @@ __global__ void unpermute_kernel(const float* __restrict__ in, const uint16_t* _
 
 }  // namespace
 
-size_t task_kernel_smem_bytes(int slots, int Hp_pad, int Ho_pad) {
+size_t task_kernel_smem_bytes(bool wide, int slots, int Hp_pad, int Ho_pad) {
     const int hx = Hp_pad > Ho_pad ? Hp_pad : Ho_pad;
-    size_t floats = size_t(9 * HCAP + 268) + size_t(slots) * hx;  // fixed-offset arrays (SM_*), then the scratch vectors
+    const int hc = 4 * (wide ? 352 : 288);  // HC of the build launch_task_kernel picks
+    size_t floats = size_t(smem_fixed_floats(hc)) + size_t(slots) * hx;  // fixed-offset arrays (SM_*), then the scratch vectors
     return floats * sizeof(float);
 }
 

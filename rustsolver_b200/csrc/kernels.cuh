@@ -123,7 +123,8 @@ struct TaskArgs {
     unsigned long long* timing;  // RS_TASK_TIMING builds: [8 kinds][count, wait cycles, body cycles, total cycles]
 };
 
-size_t task_kernel_smem_bytes(int slots, int Hp_pad, int Ho_pad);
+// dynamic shared memory of one CTA of the wide (352-thread) or the 288-thread build: the fixed arrays follow the build
+size_t task_kernel_smem_bytes(bool wide, int slots, int Hp_pad, int Ho_pad);
 // Two register specialisations of the kernel: blocks of up to 288 compute threads built for three resident CTAs per SM
 // (64 registers), and a wide one (up to 352 threads, two CTAs per SM, 80 registers).  `wide` selects the second one for a
 // block that would fit the first: a launch with too few tickets to populate a third CTA per SM is latency-bound and runs
