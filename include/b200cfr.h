@@ -283,6 +283,39 @@ int rs_set_prune_threshold(rs_engine* e, float threshold);
 #define RS_OPP_SAMPLE 1u
 #define RS_OPP_SAMPLE_TIMES_SIGMA 2u
 int rs_set_opponent_sampling(rs_engine* e, uint32_t mode, uint64_t seed);
+/* Update rule of the traverser's table update.  Let t = 1, 2, ... count the rs_iterate iterations since the rule was
+ * set or since rs_reset.  In iteration t the traverser rewrites every row of its (round, player) table as
+ *     R' = (R > 0 ? fp : fn) * R + (R > prune_threshold ? d_a : 0)      CFR_PLUS only: R' = max(R', 0)
+ *     S' = fs * S + sigma_a * w
+ * (d_a = cfv_a - cfv_node summed over the row's hands, w = the row's reach mass) with the factors of iteration t - 1
+ * (all 1 for t = 1):
+ *   RS_RULE_VANILLA   fp = fn = fs = 1 (the default, vanilla CFR)
+ *   RS_RULE_DCFR      fp = (t-1)^alpha / ((t-1)^alpha + 1), fn = (t-1)^beta / ((t-1)^beta + 1), fs = ((t-1) / t)^gamma
+ *                     (discounted CFR, Brown & Sandholm 2019; 1.5, 0, 2 are the published defaults)
+ *   RS_RULE_LCFR      DCFR with alpha = beta = gamma = 1 (linear CFR; the parameters are ignored)
+ *   RS_RULE_CFR_PLUS  fp = fn = 1, fs = (t-1) / t, regrets floored at 0 (CFR+; the parameters are ignored)
+ * The host computes each factor in double precision and rounds it to fp32.  The discount is applied lazily: a row is
+ * multiplied when its owner next updates it, with no extra pass over the tables.  It changes no strategy: regret
+ * matching reads only the positive regrets, which share one factor, and the average strategy is normalised.  The stored
+ * tables (rs_read_infoset) are the recursion above, i.e. the discounted sums lag one iteration's factor behind.  The
+ * discount_interval schedule and rs_discount scale uniformly and compose with every rule.
+ * The lazy form needs every row of the traverser's table rewritten in every iteration, which rs_iterate does (with
+ * pruning and with sampled opponent actions too).  rs_iterate_sampled does not, so it returns RS_ERR_UNSUPPORTED while a
+ * rule other than VANILLA is set; so does this call with such a rule on an engine created with RS_FLAG_STREET_KERNEL.
+ * Applies from the next iteration on; rs_reset restarts t at 1 and keeps the rule.  NaN or infinite parameters and
+ * unknown kinds are RS_ERR_INVALID.  On a board-sharded engine the call is local (not collective), but every rank must
+ * set the same rule.  rs_get_update_rule returns the rule and t of the last iteration run under it (0 before the first);
+ * either output may be NULL.  rs_profile_iteration runs an iteration too and advances t like rs_iterate. */
+#define RS_RULE_VANILLA 0u
+#define RS_RULE_DCFR 1u
+#define RS_RULE_LCFR 2u
+#define RS_RULE_CFR_PLUS 3u
+typedef struct rs_update_rule {
+    uint32_t kind; /* RS_RULE_* */
+    float alpha, beta, gamma;
+} rs_update_rule;
+int rs_set_update_rule(rs_engine* e, const rs_update_rule* rule);
+int rs_get_update_rule(rs_engine* e, rs_update_rule* out, uint64_t* t_out);
 int rs_reset(rs_engine* e);
 
 /* infoset_table[round,player][board][action node] -> [row][n_actions] (README.md:45-47).

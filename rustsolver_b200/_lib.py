@@ -54,6 +54,10 @@ class rs_stats(C.Structure):
                 ("n_hands", C.c_uint32 * 2), ("n_combos", C.c_uint64)]
 
 
+class rs_update_rule(C.Structure):
+    _fields_ = [("kind", C.c_uint32), ("alpha", C.c_float), ("beta", C.c_float), ("gamma", C.c_float)]
+
+
 class rs_kernel_time(C.Structure):
     _fields_ = [("kind", C.c_uint32), ("phase", C.c_uint32), ("traverser", C.c_uint32), ("grid", C.c_uint32),
                 ("ms", C.c_float), ("table_bytes", C.c_uint64), ("vector_bytes", C.c_uint64)]
@@ -91,6 +95,8 @@ ENGINE_API = {
     "rs_set_wait_timeout_ms": (C.c_int, [VP, C.c_uint64]),
     "rs_abort": (C.c_int, [VP]),
     "rs_sample_runouts": (C.c_int, [C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, C.c_int, u8p]),
+    "rs_set_update_rule": (C.c_int, [VP, C.POINTER(rs_update_rule)]),
+    "rs_get_update_rule": (C.c_int, [VP, C.POINTER(rs_update_rule), u64p]),
     "rs_reset": (C.c_int, [VP]),
     "rs_read_infoset": (C.c_int, [VP, C.c_uint32, C.c_uint32, f32p, f32p, C.c_size_t, u32p, u32p]),
     "rs_write_infoset": (C.c_int, [VP, C.c_uint32, C.c_uint32, f32p, f32p, C.c_size_t]),

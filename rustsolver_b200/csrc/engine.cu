@@ -6,6 +6,7 @@
 #include <cuda_runtime.h>
 #include <dlfcn.h>
 
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -209,6 +210,12 @@ struct Engine {
     bool aborted = false;             // a traversal gave up: the tables are partly updated, the engine refuses further work
     int check_abort(const char* what);
     int maybe_discount();
+    // rs_set_update_rule: the rule and t of the last iteration run under it.  VANILLA launches the plain CFR builds and
+    // writes no factors, so the default path is exactly what it was without the rule.
+    rs_update_rule rule = {RS_RULE_VANILLA, 1.5f, 0.f, 2.f};
+    uint64_t rule_t = 0;
+    bool rule_on() const { return rule.kind != RS_RULE_VANILLA; }
+    int advance_rule();
     uint64_t last_discount_period = 0;
     // fused final-street kernel (street_kernel.cu); off: the final round runs as node tasks like the others
     bool street_on = false;
@@ -412,6 +419,8 @@ int Engine::init(const rs_config* cfg) {
         c0.exited = 0;
         c0.xch_seq = 1;
         c0.epoch = 1;  // flags start at 0 = "never completed"
+        c0.rule[0] = c0.rule[1] = c0.rule[2] = 1.f;
+        c0.rule[3] = -INFINITY;
         CU(ctl.upload(&c0, 1));
         CU(cudaHostAlloc(reinterpret_cast<void**>(&abort_host), sizeof(uint32_t), cudaHostAllocMapped));
         *abort_host = 0;
@@ -776,6 +785,7 @@ int Engine::enqueue_traversal(int trav, int mode, uint64_t* count, const TaskSet
         a.xs_mode = xs_mode;
         mode = KM_CFR_XS;
     }
+    if (rule_on() && (mode == KM_CFR || mode == KM_CFR_XS)) mode = mode == KM_CFR ? KM_CFR_DR : KM_CFR_XS_DR;
     int rc;
     // Launch schedule.  Without the street kernel a traversal is one launch of the task kernel (with the in-kernel
     // exchange) or two around the NCCL all-reduce.  With it the final round's tickets [street_lo, street_hi) are
@@ -904,6 +914,10 @@ int Engine::iterate(uint64_t n) {
     }
     CU(cudaEventRecord(ev0, stream));
     for (uint64_t i = 0; i < n; ++i) {
+        {
+            int rc = advance_rule();
+            if (rc != RS_OK) return rc;
+        }
         if (use_graph) {
             CU(cudaGraphLaunch(graph_exec, stream));
             launches += launches_per_iter;
@@ -926,6 +940,35 @@ int Engine::iterate(uint64_t n) {
     CU(cudaEventElapsedTime(&ms, ev0, ev1));
     device_ms += ms;
     return check_abort("rs_iterate");
+}
+
+// Factors {fp, fn, fs, floor} of iteration t under rule r (b200cfr.h: rs_set_update_rule): those of iteration t - 1, all 1
+// for t = 1; computed in double and rounded to fp32.  x^a / (x^a + 1) is evaluated as 1 / (1 + x^-a), which stays finite
+// where x^a overflows.
+static void update_rule_factors(const rs_update_rule& r, uint64_t t, float f[4]) {
+    f[0] = f[1] = f[2] = 1.f;
+    f[3] = r.kind == RS_RULE_CFR_PLUS ? 0.f : -INFINITY;
+    if (t <= 1) return;
+    const double s = double(t - 1);
+    if (r.kind == RS_RULE_DCFR || r.kind == RS_RULE_LCFR) {
+        const bool lin = r.kind == RS_RULE_LCFR;
+        const double a = lin ? 1.0 : double(r.alpha), b = lin ? 1.0 : double(r.beta), g = lin ? 1.0 : double(r.gamma);
+        f[0] = float(1.0 / (1.0 + std::pow(s, -a)));
+        f[1] = float(1.0 / (1.0 + std::pow(s, -b)));
+        f[2] = float(std::pow(s / double(t), g));
+    } else if (r.kind == RS_RULE_CFR_PLUS) {
+        f[2] = float(s / double(t));
+    }
+}
+
+// before every rs_iterate iteration: the factors of the next t go to TaskCtl::rule on the stream (outside the graph)
+int Engine::advance_rule() {
+    if (!rule_on()) return RS_OK;
+    float f[4];
+    update_rule_factors(rule, ++rule_t, f);
+    CU(launch_set_rule(ctl.p, f, stream));
+    ++launches;
+    return RS_OK;
 }
 
 // monitor thread of train() (cfr.rs:243-262): when the iteration count crosses into a new period p = t / DISCOUNT_INTERVAL
@@ -1364,6 +1407,8 @@ int rs_iterate_sampled(rs_engine* e, const uint8_t* dealt, uint32_t n_paths) {
     if (E.aborted) return set_err(RS_ERR_CUDA, "an earlier traversal was aborted: create a new engine");
     if (P.n_rounds < 2) return set_err(RS_ERR_INVALID, "a single-street tree has no chance node to sample");
     if (P.n_sub != 1) return set_err(RS_ERR_UNSUPPORTED, "sampled iterations need one root board");
+    // a row of a board that is not sampled would miss the factors of this iteration (rs_set_update_rule)
+    if (E.rule_on()) return set_err(RS_ERR_UNSUPPORTED, "rs_iterate_sampled needs RS_RULE_VANILLA: the update rules discount rows lazily");
     if (n_paths == 0 || n_paths > P.n_boards[1]) return set_err(RS_ERR_INVALID, "n_paths must be in 1..#first-street deals");
     const uint32_t L = P.n_rounds - 1;  // cards per path
     // Board-sharded engines: every rank is handed the SAME paths (the call is collective) and keeps those whose first
@@ -1462,6 +1507,42 @@ int rs_discount(rs_engine* e, float d) {
     return RS_OK;
 }
 
+int rs_set_update_rule(rs_engine* e, const rs_update_rule* rule) {
+    if (!rule) return set_err(RS_ERR_INVALID, "null rule");
+    if (rule->kind > RS_RULE_CFR_PLUS)
+        return set_err(RS_ERR_INVALID, "kind must be RS_RULE_VANILLA (0), RS_RULE_DCFR (1), RS_RULE_LCFR (2) or RS_RULE_CFR_PLUS (3)");
+    if (!std::isfinite(rule->alpha) || !std::isfinite(rule->beta) || !std::isfinite(rule->gamma))
+        return set_err(RS_ERR_INVALID, "alpha, beta and gamma must be finite");
+    if (!e) return set_err(RS_ERR_INVALID, "null engine");
+    Engine& E = e->e;
+    if (rule->kind != RS_RULE_VANILLA && E.street_on)
+        return set_err(RS_ERR_UNSUPPORTED, "update rules other than RS_RULE_VANILLA are not available with RS_FLAG_STREET_KERNEL");
+    CU(cudaSetDevice(E.device));
+    CU(cudaStreamSynchronize(E.stream));
+    const bool was_on = E.rule_on();
+    E.rule = *rule;
+    E.rule_t = 0;
+    // the captured iteration graph launches the builds of the old rule: capture again when that changes
+    if (was_on != E.rule_on()) {
+        if (E.graph_exec) {
+            cudaGraphExecDestroy(E.graph_exec);
+            E.graph_exec = nullptr;
+        }
+        if (E.graph) {
+            cudaGraphDestroy(E.graph);
+            E.graph = nullptr;
+        }
+    }
+    return RS_OK;
+}
+
+int rs_get_update_rule(rs_engine* e, rs_update_rule* out, uint64_t* t_out) {
+    if (!e) return set_err(RS_ERR_INVALID, "null engine");
+    if (out) *out = e->e.rule;
+    if (t_out) *t_out = e->e.rule_t;
+    return RS_OK;
+}
+
 int rs_reset(rs_engine* e) {
     if (!e) return set_err(RS_ERR_INVALID, "null engine");
     Engine& E = e->e;
@@ -1474,6 +1555,7 @@ int rs_reset(rs_engine* e) {
     E.iterations = 0;
     E.device_ms = 0;
     E.launches = 0;
+    E.rule_t = 0;
     return RS_OK;
 }
 
@@ -1809,9 +1891,11 @@ int rs_profile_iteration(rs_engine* e, rs_kernel_time* out, size_t cap, uint32_t
     Engine& E = e->e;
     CU(cudaSetDevice(E.device));
     std::vector<rs_kernel_time> rec;
+    int rc = E.advance_rule();
+    if (rc != RS_OK) return rc;
     E.prof = &rec;
     uint64_t cnt = 0;
-    int rc = E.enqueue_iteration(&cnt);
+    rc = E.enqueue_iteration(&cnt);
     E.prof = nullptr;
     cudaError_t se = cudaStreamSynchronize(E.stream);
     for (size_t i = 0; i < E.prof_events.size(); ++i) {

@@ -708,10 +708,17 @@ __device__ __forceinline__ void trav_terms_or_load(const TaskArgs& A, const Ctx&
     }
 }
 
-template <int HC, int MODE, int NA>
+// Update rule (rs_set_update_rule, DR builds only): {fp, fn, fs, floor} of this iteration, read once per task.  The regret
+// update R' = max((R > 0 ? fp : fn) * R + d, floor), d already zero for a pruned action.
+__device__ __forceinline__ float4 rule_factors(const TaskArgs& A) { return ldcg4(A.ctl->rule); }
+__device__ __forceinline__ float rule_regret(const float4& f, float r, float d) { return fmaxf((r > 0.f ? f.x : f.y) * r + d, f.w); }
+
+template <int HC, int MODE, int NA, bool DR>
 __device__ __forceinline__ void task_trav(const TaskArgs& A, const Ctx& c, const NodeTask& nt, const RoundArgs& Rk, int k, int b) {
     const DevRoundPlayer& Pp = Rk.rp[c.p];
     const float scale = Rk.chance_scale[b];
+    float4 dr;
+    if (DR) dr = rule_factors(A);
     float4 v[NA];
     bool need_sd = false;
 #pragma unroll
@@ -770,8 +777,16 @@ __device__ __forceinline__ void task_trav(const TaskArgs& A, const Ctx& c, const
                 const float w = f4get(mass, i) * scale;
 #pragma unroll
                 for (int a = 0; a < NA; ++a) {
-                    g[i * NA + a] += (live && g[i * NA + a] > A.prune_threshold) ? f4get(v[a], i) - vn : 0.f;
-                    ss[i * NA + a] += live ? sg[a] * w : 0.f;
+                    if (DR) {
+                        const float r = g[i * NA + a];
+                        if (live) {
+                            g[i * NA + a] = rule_regret(dr, r, r > A.prune_threshold ? f4get(v[a], i) - vn : 0.f);
+                            ss[i * NA + a] = dr.z * ss[i * NA + a] + sg[a] * w;
+                        }
+                    } else {
+                        g[i * NA + a] += (live && g[i * NA + a] > A.prune_threshold) ? f4get(v[a], i) - vn : 0.f;
+                        ss[i * NA + a] += live ? sg[a] * w : 0.f;
+                    }
                 }
             }
         }
@@ -835,18 +850,25 @@ __device__ __forceinline__ void task_trav(const TaskArgs& A, const Ctx& c, const
             const float w = msum * scale;
 #pragma unroll
             for (int a = 0; a < NA; ++a) {
-                tabR[size_t(row) * NA + a] = rg[a] + (rg[a] > A.prune_threshold ? d[a] : 0.f);
-                tabS[size_t(row) * NA + a] = sr[a] + sg[a] * w;
+                if (DR) {
+                    tabR[size_t(row) * NA + a] = rule_regret(dr, rg[a], rg[a] > A.prune_threshold ? d[a] : 0.f);
+                    tabS[size_t(row) * NA + a] = dr.z * sr[a] + sg[a] * w;
+                } else {
+                    tabR[size_t(row) * NA + a] = rg[a] + (rg[a] > A.prune_threshold ? d[a] : 0.f);
+                    tabS[size_t(row) * NA + a] = sr[a] + sg[a] * w;
+                }
             }
         }
     }
 }
 
 // wide nodes (more than FAST_ACTIONS actions): values in shared memory, dynamic loops over the actions
-template <int HC, int MODE>
+template <int HC, int MODE, bool DR>
 __device__ __forceinline__ void task_trav_generic(const TaskArgs& A, const Ctx& c, const NodeTask& nt, const RoundArgs& Rk, int k, int b) {
     const DevRoundPlayer& Pp = Rk.rp[c.p];
     const float scale = Rk.chance_scale[b];
+    float4 dr;
+    if (DR) dr = rule_factors(A);
     const int n_act = nt.n_act;
     bool need_sd = false;
     for (int a = 0; a < n_act; ++a) {
@@ -904,8 +926,13 @@ __device__ __forceinline__ void task_trav_generic(const TaskArgs& A, const Ctx& 
                 for (int q = hs; q < he; ++q) da += V1[a * c.Hx + rpos[q]];
                 const float old = tabR[size_t(row) * n_act + a];
                 const float sga = norm > 0.f ? fmaxf(old, 0.f) * inv : uni;
-                tabS[size_t(row) * n_act + a] += sga * w;
-                tabR[size_t(row) * n_act + a] = old + (old > A.prune_threshold ? da : 0.f);
+                if (DR) {
+                    tabS[size_t(row) * n_act + a] = dr.z * tabS[size_t(row) * n_act + a] + sga * w;
+                    tabR[size_t(row) * n_act + a] = rule_regret(dr, old, old > A.prune_threshold ? da : 0.f);
+                } else {
+                    tabS[size_t(row) * n_act + a] += sga * w;
+                    tabR[size_t(row) * n_act + a] = old + (old > A.prune_threshold ? da : 0.f);
+                }
             }
         }
     }
@@ -954,8 +981,11 @@ struct TaskSlot {
     NodeTask nt;
 };
 
-template <int MODE, int MAXT, int MINB, bool XS>
+// KM: KM_CFR, KM_BR, KM_EVAL, or KM_CFR_DR (CFR with the update rule of TaskCtl::rule)
+template <int KM, int MAXT, int MINB, bool XS>
 __global__ void __launch_bounds__(MAXT + 32, MINB) task_kernel(const __grid_constant__ TaskArgs A) {
+    constexpr bool DR = KM == KM_CFR_DR;
+    constexpr int MODE = DR ? int(KM_CFR) : KM;
     constexpr int HC = 4 * MAXT;  // positions the shared-memory arrays hold
     __shared__ __align__(16) TaskSlot s_slot[2];
 
@@ -1161,11 +1191,11 @@ __global__ void __launch_bounds__(MAXT + 32, MINB) task_kernel(const __grid_cons
             }
             case TK_UP_TRAV: {
                 switch (nt.n_act) {
-                    case 2: task_trav<HC, MODE, 2>(A, c, nt, Rk, k, b); break;
-                    case 3: task_trav<HC, MODE, 3>(A, c, nt, Rk, k, b); break;
-                    case 4: task_trav<HC, MODE, 4>(A, c, nt, Rk, k, b); break;
-                    case 5: task_trav<HC, MODE, 5>(A, c, nt, Rk, k, b); break;
-                    default: task_trav_generic<HC, MODE>(A, c, nt, Rk, k, b); break;
+                    case 2: task_trav<HC, MODE, 2, DR>(A, c, nt, Rk, k, b); break;
+                    case 3: task_trav<HC, MODE, 3, DR>(A, c, nt, Rk, k, b); break;
+                    case 4: task_trav<HC, MODE, 4, DR>(A, c, nt, Rk, k, b); break;
+                    case 5: task_trav<HC, MODE, 5, DR>(A, c, nt, Rk, k, b); break;
+                    default: task_trav_generic<HC, MODE, DR>(A, c, nt, Rk, k, b); break;
                 }
                 break;
             }
@@ -1308,6 +1338,8 @@ __global__ void scale_kernel(float* __restrict__ data, size_t n, float d) {
     if (blockIdx.x == 0 && threadIdx.x < n - n4 * 4) data[n4 * 4 + threadIdx.x] *= d;
 }
 
+__global__ void set_rule_kernel(TaskCtl* ctl, float4 f) { *reinterpret_cast<float4*>(ctl->rule) = f; }
+
 __global__ void normalize_kernel(const float* __restrict__ in, float* __restrict__ out, uint32_t n_rows, uint32_t A) {
     const uint32_t row = blockIdx.x * blockDim.x + threadIdx.x;
     if (row >= n_rows) return;
@@ -1340,6 +1372,10 @@ static cudaError_t configure_for(size_t smem, int threads, int* blocks_per_sm) {
     if (e != cudaSuccess) return e;
     e = cudaFuncSetAttribute(task_kernel<KM_CFR, MAXT, MINB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
     if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(task_kernel<KM_CFR_DR, MAXT, MINB, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(task_kernel<KM_CFR_DR, MAXT, MINB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+    if (e != cudaSuccess) return e;
     e = cudaFuncSetAttribute(task_kernel<KM_BR, MAXT, MINB, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
     if (e != cudaSuccess) return e;
     e = cudaFuncSetAttribute(task_kernel<KM_EVAL, MAXT, MINB, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
@@ -1367,6 +1403,8 @@ static void launch_for(const TaskArgs& a, int mode, int grid, int threads, size_
         // one extra warp per CTA: the dispatcher
         case KM_CFR: task_kernel<KM_CFR, MAXT, MINB, false><<<grid, threads + 32, smem, st>>>(a); break;
         case KM_CFR_XS: task_kernel<KM_CFR, MAXT, MINB, true><<<grid, threads + 32, smem, st>>>(a); break;
+        case KM_CFR_DR: task_kernel<KM_CFR_DR, MAXT, MINB, false><<<grid, threads + 32, smem, st>>>(a); break;
+        case KM_CFR_XS_DR: task_kernel<KM_CFR_DR, MAXT, MINB, true><<<grid, threads + 32, smem, st>>>(a); break;
         case KM_BR: task_kernel<KM_BR, MAXT, MINB, false><<<grid, threads + 32, smem, st>>>(a); break;
         default: task_kernel<KM_EVAL, MAXT, MINB, false><<<grid, threads + 32, smem, st>>>(a); break;
     }
@@ -1386,6 +1424,11 @@ cudaError_t launch_scale(float* data, size_t n, float d, cudaStream_t st) {
     if (blocks < 1) blocks = 1;
     if (blocks > 148 * 16) blocks = 148 * 16;
     scale_kernel<<<unsigned(blocks), threads, 0, st>>>(data, n, d);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_set_rule(TaskCtl* ctl, const float f[4], cudaStream_t st) {
+    set_rule_kernel<<<1, 1, 0, st>>>(ctl, make_float4(f[0], f[1], f[2], f[3]));
     return cudaGetLastError();
 }
 

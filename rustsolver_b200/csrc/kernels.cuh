@@ -26,7 +26,9 @@ constexpr int RS_MAX_PEERS = 8;        // GPUs of one NVSwitch box
 constexpr int FAST_ACTIONS = 4;        // nodes up to this many actions keep their table rows in registers
 constexpr int MAX_TASK_THREADS = 352;  // ceil(1326 / 4) rounded up to a warp multiple
 
-enum KernelMode { KM_CFR = 0, KM_BR = 1, KM_EVAL = 2, KM_CFR_XS = 3 };  // KM_CFR_XS: CFR with per-hand sampled opponent actions
+// KM_CFR_XS: CFR with per-hand sampled opponent actions.  KM_CFR_DR / KM_CFR_XS_DR: the same with the update rule of
+// rs_set_update_rule (factors in TaskCtl::rule); the plain CFR builds carry no trace of it.
+enum KernelMode { KM_CFR = 0, KM_BR = 1, KM_EVAL = 2, KM_CFR_XS = 3, KM_CFR_DR = 4, KM_CFR_XS_DR = 5 };
 
 // Uniform number in [0, 1) of the sampled-opponent-action mode (rs_set_opponent_sampling): a counter-based hash of the
 // traversal key, the action node, the GLOBAL board id and the opponent's hand slot, so that the draw does not depend
@@ -133,6 +135,8 @@ cudaError_t configure_task_kernels(size_t smem, int threads, bool wide, int* blo
 cudaError_t launch_task_kernel(const TaskArgs& a, int mode, int grid, int threads, bool wide, size_t smem, cudaStream_t st);
 
 cudaError_t launch_scale(float* data, size_t n, float d, cudaStream_t st);
+// ctl->rule = f: one thread, the factors travel as a kernel argument so that no host buffer must outlive the call
+cudaError_t launch_set_rule(TaskCtl* ctl, const float f[4], cudaStream_t st);
 // out[row][a] = regret-matched strategy of in[row][0..A)
 cudaError_t launch_normalize(const float* in, float* out, uint32_t n_rows, uint32_t A, cudaStream_t st);
 // out[board][hand slot] = in[board][position] for the live positions of every board (out must be zeroed): root values

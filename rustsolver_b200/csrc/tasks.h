@@ -123,6 +123,10 @@ struct TaskCtl {  // device-resident dispatcher state, reset by the last CTA to 
     unsigned int abort;  // set by the first waiter that gives up (host abort word or bounded wait): every CTA leaves
     unsigned int xch_seq;  // number of the next EXCHANGING launch (board-sharded traversals): the value the exchange flags carry and
                            // the parity of the exchange buffer.  Counts the same on every rank however a traversal is cut into launches
+    // Update-rule factors of the current iteration (rs_set_update_rule): {fp, fn, fs, floor}, floor = 0 (CFR+) or -inf.
+    // Only the KM_CFR_DR builds read them.  Graph replay fixes kernel arguments, so they live here, next to the state the
+    // kernel already reaches through TaskArgs::ctl; the engine rewrites them on its stream before every iteration.
+    alignas(16) float rule[4];
 };
 
 }  // namespace rs

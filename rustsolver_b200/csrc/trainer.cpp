@@ -140,6 +140,10 @@ MCCFRTrainer* MCCFRTrainer::init(const Options& options, const TrainerConfig& cf
         if (err) *err = rs_last_error();
         return nullptr;
     }
+    if (cfg.update_rule.kind != RS_RULE_VANILLA && rs_set_update_rule(t->engine_, &cfg.update_rule) != RS_OK) {
+        if (err) *err = rs_last_error();
+        return nullptr;
+    }
     return t.release();
 }
 

@@ -35,6 +35,8 @@ struct TrainerConfig {
     uint8_t nccl_id[RS_NCCL_ID_BYTES] = {0};
     uint32_t flags = 0;
     uint64_t discount_interval = 0, discount_cap = 0;
+    // update rule of the table update (rs_set_update_rule); RS_RULE_VANILLA is train()'s plain CFR
+    rs_update_rule update_rule = {RS_RULE_VANILLA, 1.5f, 0.f, 2.f};
     // card_abs vector of MCCFRTrainer::init (cfr.rs:167-172): one entry per betting round
     std::vector<uint32_t> abs_kind;
     std::vector<std::vector<uint32_t>> cluster_arr;  // per round, for EMD / OCHS

@@ -20,13 +20,14 @@ import numpy as np
 
 from . import _lib
 from ._lib import (EngineError, check, f32p, f64p, i32p, rs_abstraction, rs_config, rs_ranges,
-                   rs_round_abstraction, rs_stats, rs_tree, u8p, u16p, u32p, u64p)
+                   rs_round_abstraction, rs_stats, rs_tree, rs_update_rule, u8p, u16p, u32p, u64p)
 
 RS_ABS_NONE, RS_ABS_ISOMORPHIC, RS_ABS_CLUSTER_ARR, RS_ABS_BUCKET_TABLE = 0, 1, 2, 3
 RS_FLAG_NO_GRAPH = 1
 RS_FLAG_NO_CHAIN_SPLIT = 2
 RS_FLAG_STREET_KERNEL = 4
 RS_FLAG_SHARD_ISOLATED = 8
+RS_RULE_VANILLA, RS_RULE_DCFR, RS_RULE_LCFR, RS_RULE_CFR_PLUS = 0, 1, 2, 3
 NODE_ACTION, NODE_TERMINAL, NODE_PUBLIC_CHANCE, NODE_PRIVATE_CHANCE = 0, 1, 2, 3
 TERM_ALLIN, TERM_SHOWDOWN, TERM_UNCONTESTED = 0, 1, 2
 ACTION_NAMES = {0: "Bet", 1: "Raise", 2: "Check", 3: "Call", 4: "Fold"}
@@ -659,6 +660,18 @@ class Engine(_PlanOrEngine):
         """mccfr()'s opponent arm for every hand at once (cfr.rs:466-475): 0 = off, 1 = one sampled action per opponent
         hand and node keeps the whole reach, 2 = keeps reach * sigma(sampled action) as the reference's code does."""
         check(self._lib.rs_set_opponent_sampling(self._h, int(mode), int(seed)))
+
+    def set_update_rule(self, kind: int, alpha: float = 1.5, beta: float = 0.0, gamma: float = 2.0):
+        """Update rule of the traverser's table update from the next iteration on (rs_set_update_rule): RS_RULE_VANILLA,
+        RS_RULE_DCFR(alpha, beta, gamma), RS_RULE_LCFR or RS_RULE_CFR_PLUS.  Restarts the rule's iteration count t."""
+        r = rs_update_rule(int(kind), float(alpha), float(beta), float(gamma))
+        check(self._lib.rs_set_update_rule(self._h, C.byref(r)))
+
+    def update_rule(self):
+        """-> (kind, alpha, beta, gamma, t): the rule and t of the last iteration run under it."""
+        r, t = rs_update_rule(), C.c_uint64()
+        check(self._lib.rs_get_update_rule(self._h, C.byref(r), C.byref(t)))
+        return r.kind, r.alpha, r.beta, r.gamma, int(t.value)
 
     def set_wait_timeout_ms(self, ms: int):
         """Bound of every wait inside the traversal kernel (default 30 s, 0 = unbounded): see rs_set_wait_timeout_ms."""
